@@ -1,13 +1,15 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the monai_b200 hot path (sliding-window inference, voxels/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload unet_c2|swin_c3] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload unet_c2|swin_c3] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one full `SlidingWindowInferer(...)(volume, network)` pass over one synthetic volume.
   value : voxels/s with the volume already resident in HBM (CUDA-event timed, max over ranks)
   e2e   : the same call with a pinned HOST volume: H2D copy + inference + D2H copy of the logits inside the timed region
   roofline / cpu_baseline / clocks / gpu_launches : see DESIGN.md "Measurement"
 `--impl reference` times the reference algorithm's CPU path (the oracle port: torch-CPU restatement, all host threads).
+`--dump-outputs DIR` writes what the last timed step returned as DIR/<name>.npy (see dump_outputs); inputs and weights are seeded,
+so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -52,6 +54,22 @@ WORKLOADS = {
         vol=(256, 256, 256), volumes=32, net=None,
     ),
 }
+
+
+DUMP_BUDGET = 32 << 20   # bytes that --dump-outputs writes, all arrays together
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each output as <out_dir>/<name>.npy in float32.  An output with more elements than its share of DUMP_BUDGET allows is
+    written as its values at a fixed sample of flat indices, torch.randint(numel, (n,), generator=torch.Generator().manual_seed(0))."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BUDGET // 4 // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach().as_subclass(torch.Tensor)
+        if t.numel() > share:
+            idx = torch.randint(t.numel(), (share,), generator=torch.Generator().manual_seed(0))
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.float().cpu().numpy())
 
 
 def _quiet_nccl() -> None:
@@ -275,9 +293,7 @@ def run_transforms(args, wl):
     out_host = None
 
     def step_resident():
-        for v in dev_vols:
-            y = pipe({"image": MetaTensor(v, affine=aff)})["image"]
-        return y
+        return [pipe({"image": MetaTensor(v, affine=aff)})["image"] for v in dev_vols]
 
     def step_e2e():
         nonlocal out_host
@@ -289,6 +305,7 @@ def run_transforms(args, wl):
         return y
 
     def timed(fn, steps, warmup):
+        """Milliseconds of `steps` timed calls of fn and what the last one returned."""
         for _ in range(warmup):
             fn()
         torch.cuda.synchronize()
@@ -297,10 +314,11 @@ def run_transforms(args, wl):
         torch.cuda.synchronize()
         ms = 0.0
         for _ in range(steps):
+            out = None   # a step's result is released before the next step runs
             flush.fill_(1)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            fn()
+            out = fn()
             e1.record()
             e1.synchronize()
             ms += e0.elapsed_time(e1)
@@ -310,20 +328,23 @@ def run_transforms(args, wl):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms
+        return ms, out
 
     sampler = ClockSampler(local) if rank == 0 else None
     l0 = _lib.launch_count()
-    ms_total = timed(step_resident, args.steps, args.warmup)
+    ms_total, ys = timed(step_resident, args.steps, args.warmup)
     launches = (_lib.launch_count() - l0) * args.steps // (args.steps + args.warmup)
     clocks = sampler.stop() if sampler else {}
-    ms_e2e = timed(step_e2e, args.steps, 1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {f"image_{i:02d}": y for i, y in enumerate(ys)})
+    del ys
+    ms_e2e, _ = timed(step_e2e, args.steps, 1)
     K.profile_start()
-    y = step_resident()
+    y = step_resident()[-1]
     prof = K.profile_stop()
     # the same pipeline with Compose(lazy=True): reported next to the eager (reference default) number, not instead of it
     eager_pipe, pipe = pipe, _transform_pipeline(lazy=True)
-    ms_lazy = timed(step_resident, args.steps, 1)
+    ms_lazy, _ = timed(step_resident, args.steps, 1)
     pipe = eager_pipe
     if rank != 0:
         if dist is not None:
@@ -387,7 +408,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--sw-batch", type=int, default=0, help="override the workload's sw_batch_size")
     ap.add_argument("--no-secondary", action="store_true", help="skip the C2 / C4 lines appended to the default single-GPU run")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step of the workload's GPU path as DIR/<name>.npy "
+                    f"(float32, at most {DUMP_BUDGET >> 20} MiB in all: larger outputs as a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if os.environ.get("B200_BENCH_WATCHDOG"):
         import faulthandler
 
@@ -473,6 +500,7 @@ def main():
         return y
 
     def timed(fn, steps, warmup):
+        """Milliseconds of `steps` timed calls of fn and what the last one returned."""
         for _ in range(warmup):
             fn()
         torch.cuda.synchronize()
@@ -481,10 +509,11 @@ def main():
         torch.cuda.synchronize()
         ms = 0.0
         for _ in range(steps):
+            out = None   # a step's result is released before the next step runs
             flush.fill_(1)  # L2 flush between timed iterations (untimed)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            fn()
+            out = fn()
             e1.record()
             e1.synchronize()
             ms += e0.elapsed_time(e1)
@@ -494,14 +523,17 @@ def main():
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms
+        return ms, out
 
     sampler = ClockSampler(local) if rank == 0 else None
     l0 = _lib.launch_count()
-    ms_total = timed(step_resident, args.steps, args.warmup)
+    ms_total, y = timed(step_resident, args.steps, args.warmup)
     launches = (_lib.launch_count() - l0) * args.steps // (args.steps + args.warmup)
     clocks = sampler.stop() if sampler else {}
-    ms_e2e = timed(step_e2e, args.steps, 1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"logits": y})
+    del y
+    ms_e2e, _ = timed(step_e2e, args.steps, 1)
 
     # per-kernel device time (CUDA events around every C-ABI launch, one extra untimed-for-value pass)
     K.profile_start()   # CUDA-graph replay is bypassed while profiling so every launch is individually timed

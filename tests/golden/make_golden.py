@@ -328,6 +328,21 @@ def grid_pull_ref():
     save("grid_pull.npz", **out)
 
 
+def grid_pull_ref_dst2():
+    """monai._C.grid_pull of the REAL reference (oracle/_ref, CPU), dst2 bound, cubic order, samples outside the field of view:
+    the inputs of tests/test_oracle_resample.py::test_oracle_matches_the_stored_compiled_reference_dst2_cubic (seeded the same way)."""
+    sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+    from oracle import build_ref
+
+    C = build_ref.load()
+    assert C is not None, "run python oracle/build_ref.py first"
+    rng = np.random.default_rng(0)
+    x = rng.standard_normal((1, 2, 5, 4, 6)).astype(np.float32)
+    grid = (rng.random((1, 3, 4, 5, 3)) * 9 - 2).astype(np.float32)
+    y = C.grid_pull(torch.from_numpy(x), torch.from_numpy(grid), [C.BoundType(4)] * 3, [C.InterpolationType(3)] * 3, True).numpy()
+    save("grid_pull_dst2_cubic.npz", x=x, grid=grid, y=y)
+
+
 def grid_push_ref():
     """monai._C.grid_push / grid_count of the REAL reference (oracle/_ref, CPU): random coordinates reaching outside the field of
     view, the seven bounds, orders 0-3, extrapolate on / off; the numpy restatement (oracle/resample.py) is checked on all 56
@@ -640,6 +655,6 @@ def unit_goldens():
 
 if __name__ == "__main__":
     print("reference monai", monai.__version__, "torch", torch.__version__)
-    which = sys.argv[1:] or ["planner", "sliding", "nets", "nets_r2", "dynunet", "segresnet", "unetr", "buffered", "resampler", "grid_pull_ref", "grid_push_ref", "lazy_inverse", "transforms", "post", "patch", "unit_goldens"]
+    which = sys.argv[1:] or ["planner", "sliding", "nets", "nets_r2", "dynunet", "segresnet", "unetr", "buffered", "resampler", "grid_pull_ref", "grid_pull_ref_dst2", "grid_push_ref", "lazy_inverse", "transforms", "post", "patch", "unit_goldens"]
     for w in which:
         globals()[w]()

@@ -3,7 +3,6 @@ of the reference's own C++ sources (compiled into oracle/_ref by oracle/build_re
 import os
 
 import numpy as np
-import pytest
 
 from oracle import resample as ors
 
@@ -34,20 +33,25 @@ def test_oracle_matches_compiled_reference_3d(golden_dir):
     np.testing.assert_allclose(ors.grid_pull(g["x"], g["grid"], [0, 0, 0], [1, 1, 1], extrapolate=False), g["y.noextrap"], rtol=2e-4, atol=2e-5)
 
 
-def test_compiled_reference_loads_when_present():
-    """oracle/_ref travels with the snapshot: when the .so is there it must import and agree with the restatement."""
-    from oracle import build_ref
-
-    C = build_ref.load()
-    if C is None:
-        pytest.skip("oracle/_ref has not been built on this box")
-    import torch
-
+def test_oracle_matches_the_stored_compiled_reference_dst2_cubic(golden_dir):
+    """monai._C.grid_pull of the reference's own C++ (dst2, cubic; fixture of make_golden.py grid_pull_ref_dst2) against the
+    restatement.  Where oracle/_ref has been built, the compiled module must also import and reproduce the stored output."""
+    g = np.load(os.path.join(golden_dir, "grid_pull_dst2_cubic.npz"))
     rng = np.random.default_rng(0)
     x = rng.standard_normal((1, 2, 5, 4, 6)).astype(np.float32)
     grid = (rng.random((1, 3, 4, 5, 3)) * 9 - 2).astype(np.float32)
-    ref = C.grid_pull(torch.from_numpy(x), torch.from_numpy(grid), [C.BoundType(4)] * 3, [C.InterpolationType(3)] * 3, True).numpy()
-    np.testing.assert_allclose(ors.grid_pull(x, grid, [4] * 3, [3] * 3), ref, rtol=2e-4, atol=2e-5)
+    np.testing.assert_array_equal(x, g["x"])
+    np.testing.assert_array_equal(grid, g["grid"])
+    np.testing.assert_allclose(ors.grid_pull(x, grid, [4] * 3, [3] * 3), g["y"], rtol=2e-4, atol=2e-5)
+
+    from oracle import build_ref
+
+    C = build_ref.load()
+    if C is not None:
+        import torch
+
+        ref = C.grid_pull(torch.from_numpy(x), torch.from_numpy(grid), [C.BoundType(4)] * 3, [C.InterpolationType(3)] * 3, True).numpy()
+        np.testing.assert_allclose(ref, g["y"], rtol=1e-6, atol=1e-6)
 
 
 def test_oracle_push_and_count_match_the_compiled_reference(golden_dir):
